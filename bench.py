@@ -33,6 +33,7 @@ import sys
 import threading
 import time
 
+import numpy as np
 import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
@@ -65,7 +66,12 @@ def parse_args():
                     help="skip timing the reference's own layer classes on its own CUDA kernels (frames.reference_stack)")
     ap.add_argument("--frames-steps", type=int, default=5)
     ap.add_argument("--cpu-budget-s", type=float, default=25.0, help="target CPU seconds for the cpu_baseline sample")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned (rank 0) as DIR/<call>_<name>.npy; see dump_outputs()")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 def dist_env():
@@ -195,7 +201,7 @@ def run_b200(args):
         return (c["value"], c["spatial_shapes"], c["level_start_index"], c["sampling_locations"],
                 c["attention_weights"])
 
-    def step(ev=None):
+    def step(ev=None, keep=None):
         for i, c in enumerate(calls):
             a = op_args(c)
             if ev is not None:
@@ -206,6 +212,8 @@ def run_b200(args):
             grads = MSDA.ms_deform_attn_backward(*a, c["grad_output"], 64)
             if ev is not None:
                 ev[i][2].record()
+            if keep is not None:
+                keep.append((out, *grads))
         return out, grads
 
     def barrier():
@@ -214,8 +222,9 @@ def run_b200(args):
             dist.barrier()
         torch.cuda.synchronize()
 
+    dump = args.dump_outputs is not None and rank == 0
     for _ in range(max(3, args.warmup)):
-        step()
+        step(keep=[] if dump else None)    # when dumping, warm-up holds a step's results too: same allocator pool as the last timed step
     barrier()
 
     # ---- timed region: exactly K steps, device-resident inputs ----
@@ -228,12 +237,16 @@ def run_b200(args):
         time.sleep(0.25)
     barrier()
     launches0 = lib.msda_launch_count()
+    last = [] if dump else None
     t0.record()
     for k in range(K):
-        step(evs[k])
+        step(evs[k], keep=last if k == K - 1 else None)
     t1.record()
     barrier()
     launches = lib.msda_launch_count() - launches0
+    if dump:
+        dump_outputs(args.dump_outputs, calls, last)
+        del last
     total_ms = t0.elapsed_time(t1)
     clocks = sampler.stop() if rank == 0 else None
     if world > 1:
@@ -318,6 +331,29 @@ def run_b200(args):
     if world > 1:
         import torch.distributed as dist
         dist.destroy_process_group()
+
+
+DUMP_ELEMS = 1 << 18      # per array: 12 calls x 4 arrays x 1 MB (float32) stay below 64 MB
+
+
+def dump_outputs(path, calls, results):
+    """Writes the arrays the timed path returned to its caller in the last timed step: for every call (enc0..enc5,
+    dec0..dec5) ``out``, ``grad_value``, ``grad_loc`` and ``grad_attn`` as ``<call>_<name>.npy`` in float32 (bf16 results
+    widened).  An array of more than DUMP_ELEMS elements is stored as a fixed sample: the flattened elements at indices
+    i * 2654435761 mod numel for i < DUMP_ELEMS, ascending -- the same elements in every run, since the multiplier is a
+    prime larger than any array here.  Inputs are seeded, so two builds run with the same arguments compare element for
+    element: out, grad_loc and grad_attn repeat bit for bit, grad_value (accumulated with atomics) to rounding."""
+    os.makedirs(path, exist_ok=True)
+    counts = {"enc": 0, "dec": 0}
+    for c, arrays in zip(calls, results):
+        call = f"{c['kind']}{counts[c['kind']]}"
+        counts[c["kind"]] += 1
+        for name, t in zip(("out", "grad_value", "grad_loc", "grad_attn"), arrays):
+            flat = t.detach().reshape(-1)
+            if flat.numel() > DUMP_ELEMS:
+                idx = torch.arange(DUMP_ELEMS, dtype=torch.int64, device=flat.device) * 2654435761 % flat.numel()
+                flat = flat[idx.sort().values]
+            np.save(os.path.join(path, f"{call}_{name}.npy"), flat.float().cpu().numpy())
 
 
 def _time_call(fn, iters=10, warm=3):
@@ -506,21 +542,20 @@ def build_reference_stack(cfg, tr_mod, num_layers=6, d_ffn=2048):
 def reference_stack_leg(cfg, device, steps, lib, inputs, ours):
     """The anchor for frames/s: the SAME step (6 + 6 layers fwd + bwd, same synthetic features, same loss) run by the
     REFERENCE's GPU stack -- its own Python classes (``DeformableTransformerEncoderLayer`` / ``DecoderLayer`` /
-    ``MSDeformAttn`` / ``MSDeformAttnFunction`` of deformable_transformer.py and ops/, unmodified files staged in tests/_ref)
+    ``MSDeformAttn`` / ``MSDeformAttnFunction`` of deformable_transformer.py and ops/, unmodified files staged in oracle/_ref/py)
     on its own CUDA kernels (ms_deform_im2col_cuda.cuh compiled unmodified into oracle/_ref/libmsda_refcuda.so).  None of
     this repo's kernels is on that path (checked with the library's launch counter).  Baseline leg only, outside every
     timed region of this repo's numbers, like `reference_cuda`."""
     try:
-        from oracle import refcuda
-        from tests import stage_reference
-        if not stage_reference.staged():
-            return {"unavailable": "tests/_ref not staged (needs /root/reference at build time)"}
+        from oracle import refcuda, refstage
+        if not refstage.staged():
+            return {"unavailable": "oracle/_ref/py not staged (needs a reference checkout at build time)"}
         if not refcuda.available():
             return {"unavailable": "oracle/_ref/libmsda_refcuda.so not built (needs /root/reference at build time)"}
         import warnings
         with warnings.catch_warnings():
             warnings.simplefilter("ignore")
-            func_mod, _attn_mod, tr_mod, _dino_mod = stage_reference.import_reference()
+            func_mod, _attn_mod, tr_mod, _dino_mod = refstage.import_reference()
 
         src, pos, shapes, ss, lsi, pad = inputs
         model = build_reference_stack(cfg, tr_mod).to(device)
@@ -549,7 +584,7 @@ def reference_stack_leg(cfg, device, steps, lib, inputs, ours):
                         "msda_b200_launches_per_step": int((lib.msda_launch_count() - l0) / steps)}
 
             res = {"what": "the reference's own layer classes (deformable_transformer.py:321-416, ops/modules, ops/functions; "
-                           "unmodified files, tests/_ref) on the reference's own CUDA kernels (oracle/_ref), eager PyTorch as "
+                           "unmodified files, oracle/_ref/py) on the reference's own CUDA kernels (oracle/_ref), eager PyTorch as "
                            "the reference runs them; same step, features and loss as the legs above; single GPU"}
             old = torch.backends.cuda.matmul.allow_tf32
             try:

@@ -32,11 +32,6 @@ def pytest_sessionstart(session):
         _o.build()
     except Exception as exc:                       # no nvcc / gcc here: the tests that need the libraries will say so
         print(f"[conftest] native build skipped: {exc}")
-    try:                                           # reference Python files for the "reference classes on the drop-in" tests
-        from tests import stage_reference          # (copies only where /root/reference exists; git-ignored tests/_ref)
-        stage_reference.stage()
-    except Exception as exc:
-        print(f"[conftest] reference staging skipped: {exc}")
 
 
 def golden_names():

@@ -1,103 +1,62 @@
 """GPU tests (-m gpu) of the CondInst dynamic mask head (uninext_b200/modules/dynamic_mask_head.py, kernels in
 csrc/msda_condinst.cuh) against the REFERENCE functions themselves -- ``DDETRSegmUni.dynamic_mask_with_coords`` /
-``mask_heads_forward`` / ``parse_dynamic_params`` / ``aligned_bilinear`` / ``compute_locations`` from the staged copy of
-uninext/models/ddetrs.py (tests/stage_reference.py), run on the GPU with grouped convolutions: forward and every
-gradient (mask features, dynamic parameters, reference points), fp32, 2e-4 of scale."""
-import types
-import warnings
-
+``mask_heads_forward`` / ``parse_dynamic_params`` / ``aligned_bilinear`` / ``compute_locations`` of
+uninext/models/ddetrs.py, whose fp32 results on the same inputs are stored under tests/golden/reference
+(tests/reference_cases.py, tests/golden/make_reference_golden.py): forward and every gradient (mask features, dynamic
+parameters, reference points), fp32, 2e-4 of scale."""
 import pytest
 import torch
 
-from tests import stage_reference
+from tests import reference_cases as rc
 
-pytestmark = [pytest.mark.gpu,
-              pytest.mark.skipif(not stage_reference.staged(), reason="tests/_ref not staged (python tests/stage_reference.py)")]
+pytestmark = pytest.mark.gpu
 
 if torch.cuda.is_available():
     from uninext_b200 import _cabi
-    from uninext_b200.modules.dynamic_mask_head import (CondInstMaskHead, aligned_bilinear, dynamic_mask_with_coords,
-                                                        dynamic_param_counts)
+    from uninext_b200.modules.dynamic_mask_head import CondInstMaskHead, aligned_bilinear, dynamic_mask_with_coords
 
 DEV = "cuda"
 
 
 @pytest.fixture(scope="module")
-def ddetrs():
-    with warnings.catch_warnings():
-        warnings.simplefilter("ignore")
-        return stage_reference.import_ddetrs()
-
-
-@pytest.fixture(autouse=True)
-def _strict_fp32_reference():
-    """The reference runs its dynamic layers as cuDNN grouped convolutions, which default to TF32 on this GPU; the parity
-    bar is fp32, so the reference side is pinned to fp32 convolutions for these tests."""
-    old = torch.backends.cudnn.allow_tf32
-    torch.backends.cudnn.allow_tf32 = False
-    yield
-    torch.backends.cudnn.allow_tf32 = old
-
-
-def _rel(got, want):
-    return ((got.detach().double() - want.detach().double()).abs().max() / want.detach().double().abs().max().clamp_min(1e-30)).item()
-
-
-def _holder(ddetrs, rel_coord, mask_out_stride):
-    """An object with exactly the attributes the reference method reads (ddetrs.py:45-70)."""
-    h = types.SimpleNamespace(dynamic_mask_channels=8, mask_out_stride=mask_out_stride, use_raft=False)
-    h.weight_nums, h.bias_nums = dynamic_param_counts(3, rel_coord)
-    h.mask_heads_forward = lambda *a: ddetrs.DDETRSegmUni.mask_heads_forward(h, *a)
-    return h
+def aligned_golden():
+    return rc.load("condinst_aligned")
 
 
 @pytest.mark.parametrize("factor", [2, 4])
 @pytest.mark.parametrize("shape", [(3, 5, 7), (2, 1, 1), (1, 13, 21), (5, 40, 66)])
-def test_aligned_bilinear_matches_reference(ddetrs, factor, shape):
-    g = torch.Generator().manual_seed(1)
-    x = torch.randn(*shape, generator=g).to(DEV)
+def test_aligned_bilinear_matches_reference(aligned_golden, factor, shape):
+    x, g = rc.aligned_inputs(shape, DEV)
     a = x.clone().requires_grad_(True)
-    b = x.clone().requires_grad_(True)
-    want = ddetrs.aligned_bilinear(b[None], factor)[0]
     got = aligned_bilinear(a, factor)
-    assert got.shape == want.shape and _rel(got, want) < 1e-6
-    go = torch.randn(want.shape, generator=g).to(DEV)
-    got.backward(go); want.backward(go)
-    assert _rel(a.grad, b.grad) < 1e-5
+    cid = rc.aligned_id(factor, shape)
+    assert rc.rel_err(got, aligned_golden, cid + "/out") < 1e-6
+    go = torch.randn(got.shape, generator=g).to(DEV)
+    got.backward(go)
+    assert rc.rel_err(a.grad, aligned_golden, cid + "/grad") < 1e-5
 
 
 @pytest.mark.parametrize("rel_coord", [True, False])
 @pytest.mark.parametrize("num_insts,hw,mask_out_stride", [([5, 3], (12, 20), 4), ([0, 7], (9, 11), 4), ([37, 21, 1], (25, 42), 8),
                                                           ([300], (32, 40), 4), ([30, 17], (100, 168), 4), ([3], (7, 9), 2)])
-def test_dynamic_mask_head_matches_reference(ddetrs, rel_coord, num_insts, hw, mask_out_stride):
-    g = torch.Generator().manual_seed(2)
-    n, (h, w), total = len(num_insts), hw, sum(num_insts)
-    npar = sum(sum(x) for x in dynamic_param_counts(3, rel_coord))
-    feats = torch.randn(n, 8, h, w, generator=g).to(DEV)
-    refs = (torch.rand(1, total, 2, generator=g) * torch.tensor([w * 8.0, h * 8.0])).to(DEV)
-    params = (torch.randn(1, total, npar, generator=g) * 0.3).to(DEV)
-    leaves = lambda: [t.clone().requires_grad_(True) for t in (feats, refs, params)]
-    fa, ra, pa = leaves()
-    fb, rb, pb = leaves()
+def test_dynamic_mask_head_matches_reference(rel_coord, num_insts, hw, mask_out_stride):
+    feats, refs, params, g = rc.dynamic_inputs(rel_coord, num_insts, hw, DEV)
+    want = rc.load(rc.dynamic_id(rel_coord, num_insts, hw, mask_out_stride))
+    fa, ra, pa = (t.clone().requires_grad_(True) for t in (feats, refs, params))
     lib = _cabi.load()
     before = lib.msda_launch_count()
     got = dynamic_mask_with_coords(fa, ra, pa, num_insts, 8, rel_coord, mask_out_stride)
     assert lib.msda_launch_count() > before
-    with warnings.catch_warnings():
-        warnings.simplefilter("ignore")
-        want = ddetrs.DDETRSegmUni.dynamic_mask_with_coords(_holder(ddetrs, rel_coord, mask_out_stride), fb, rb, pb,
-                                                            num_insts=num_insts, mask_feat_stride=8, rel_coord=rel_coord)
-    assert got.shape == want.shape
-    assert _rel(got, want) < 2e-4
-    go = torch.randn(want.shape, generator=g).to(DEV)
-    got.backward(go); want.backward(go)
-    assert _rel(fa.grad, fb.grad) < 2e-4
-    assert _rel(pa.grad, pb.grad) < 2e-4
+    assert rc.rel_err(got, want, "out") < 2e-4
+    go = torch.randn(got.shape, generator=g).to(DEV)
+    got.backward(go)
+    assert rc.rel_err(fa.grad, want, "grad_feats") < 2e-4
+    assert rc.rel_err(pa.grad, want, "grad_params") < 2e-4
     if rel_coord:
-        assert _rel(ra.grad, rb.grad) < 1e-3            # piecewise-linear through two ReLUs: sums of many signed terms
+        assert rc.rel_err(ra.grad, want, "grad_refs") < 1e-3      # piecewise-linear through two ReLUs: sums of many signed terms
 
 
-def test_condinst_module_parameter_names_and_forward(ddetrs):
+def test_condinst_module_parameter_names_and_forward():
     torch.manual_seed(3)
     head = CondInstMaskHead(256).to(DEV)
     assert set(head.state_dict()) == {f"controller.layers.{i}.{k}" for i in range(3) for k in ("weight", "bias")}

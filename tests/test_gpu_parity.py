@@ -291,27 +291,26 @@ def test_reference_gradcheck_fp64(channels):
 
 
 # ---------------------------------------------------------------------------------------------------------------
-# (5) against the reference's own CUDA kernels (oracle/_ref, built from /root/reference by oracle/build_refcuda.sh)
+# (5) against the reference's own CUDA kernels (ms_deform_im2col_cuda.cuh compiled unmodified for sm_100a; their
+#     results on these inputs are stored under tests/golden/reference by tests/golden/make_reference_golden.py --refcuda)
 # ---------------------------------------------------------------------------------------------------------------
 @pytest.mark.parametrize("cfgname,kind,dtype", [("cfg1", "enc", torch.float32), ("cfg2", "enc", torch.float32),
                                                 ("cfg2", "dec", torch.float32), ("cfg1", "dec", torch.float64)])
 def test_against_reference_cuda_kernels(cfgname, kind, dtype):
-    from oracle import refcuda
-    if not refcuda.available():
-        pytest.skip("oracle/_ref/libmsda_refcuda.so not built (needs /root/reference at build time)")
+    from tests import reference_cases as rc
+    want = rc.load(f"refcuda_{cfgname}_{kind}_{'f32' if dtype == torch.float32 else 'f64'}")
     inp = make_inputs(CONFIGS[cfgname], kind, DEV, dtype=dtype, seed=13, wild_fraction=0.05)
+    sums = [float(inp[k].double().sum()) for k in ("value", "sampling_locations", "attention_weights", "grad_output")]
+    np.testing.assert_allclose(sums, want["input_sums"], rtol=1e-9, err_msg="inputs differ from the stored case")
     a = (inp["value"], inp["spatial_shapes"], inp["level_start_index"], inp["sampling_locations"],
          inp["attention_weights"])
-    ref_out = refcuda.forward(*a)
-    ref_gv, ref_gl, ref_ga = refcuda.backward(*a, inp["grad_output"])
     out = MSDA.ms_deform_attn_forward(*a, 64)
     gv, gl, ga = MSDA.ms_deform_attn_backward(*a, inp["grad_output"], 64)
     tol = 1e-4 if dtype == torch.float32 else 1e-11
-    rel = lambda x, y: ((x - y).abs().max() / y.abs().max().clamp_min(1e-30)).item()
-    assert rel(out, ref_out) < tol
-    assert rel(gv, ref_gv) < tol
-    assert rel(gl, ref_gl) < 2 * tol
-    assert rel(ga, ref_ga) < tol
+    assert rc.rel_err(out, want, "out") < tol
+    assert rc.rel_err(gv, want, "grad_value") < tol
+    assert rc.rel_err(gl, want, "grad_loc") < 2 * tol
+    assert rc.rel_err(ga, want, "grad_attn") < tol
 
 
 # ---------------------------------------------------------------------------------------------------------------

@@ -1,6 +1,6 @@
 """CPU test of bench.py's `frames.reference_stack` wiring (no GPU): the reference's own layer classes (files staged in
-tests/_ref) dropped into run_frames' stack run forward + backward when ``ms_deform_attn_func.MSDA`` is rebound to a
-kernels module -- here one built on the reference's CPU function instead of oracle/_ref's CUDA kernels."""
+oracle/_ref/py by build() from a reference checkout; skipped without one) dropped into run_frames' stack run forward +
+backward when ``ms_deform_attn_func.MSDA`` is rebound to a kernels module -- here one built on the reference's CPU function instead of oracle/_ref's CUDA kernels."""
 import os
 import sys
 import warnings
@@ -11,9 +11,9 @@ import torch
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 
-from tests import stage_reference  # noqa: E402
+from oracle import refstage  # noqa: E402
 
-pytestmark = pytest.mark.skipif(not stage_reference.stage(), reason="tests/_ref not staged (no /root/reference here)")
+pytestmark = pytest.mark.skipif(not refstage.staged(), reason="oracle/_ref/py not staged (no reference checkout at build time)")
 
 
 class _CpuKernels:
@@ -38,7 +38,7 @@ def test_reference_layers_run_inside_the_bench_stack():
     from uninext_b200.workloads import OpConfig, level_tensors
     with warnings.catch_warnings():
         warnings.simplefilter("ignore")
-        func_mod, _attn, tr_mod, _dino = stage_reference.import_reference()
+        func_mod, _attn, tr_mod, _dino = refstage.import_reference()
     cfg = OpConfig("tiny", 64, 64, 2, 10)
     shapes = cfg.shapes
     model = bench.build_reference_stack(cfg, tr_mod, num_layers=2, d_ffn=64)

@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """CondInst dynamic mask head: this repo's fused kernels vs the REFERENCE function (staged uninext/models/ddetrs.py:
 repeat + three grouped convolutions + aligned_bilinear) on the same B200, forward and forward+backward.
-    python tools/condinst_bench.py          (needs tests/_ref staged: python tests/stage_reference.py)"""
+    python tools/condinst_bench.py          (needs oracle/_ref/py staged: python -m oracle.refstage)"""
 import json
 import os
 import sys
@@ -11,12 +11,12 @@ import warnings
 import torch
 
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-from tests import stage_reference  # noqa: E402
+from oracle import refstage  # noqa: E402
 from uninext_b200.modules.dynamic_mask_head import dynamic_mask_with_coords, dynamic_param_counts  # noqa: E402
 
 with warnings.catch_warnings():
     warnings.simplefilter("ignore")
-    ddetrs = stage_reference.import_ddetrs()
+    ddetrs = refstage.import_ddetrs()
 h = types.SimpleNamespace(dynamic_mask_channels=8, mask_out_stride=4, use_raft=False)
 h.weight_nums, h.bias_nums = dynamic_param_counts(3, True)
 h.mask_heads_forward = lambda *a: ddetrs.DDETRSegmUni.mask_heads_forward(h, *a)
