@@ -32,7 +32,11 @@
  *     accumulation is fp32.
  *   - backward: grad_value is zero-filled by the callee (the reference's at::zeros_like, cu:121); grad_sampling_loc
  *     and grad_attn_weight are fully overwritten. grad_value accumulation order is not deterministic (fp32 atomics),
- *     like the reference.
+ *     like the reference: grad_value agrees between runs only to rounding.  grad_sampling_loc and grad_attn_weight are
+ *     run-to-run stable for a given kernel selection; the forward has no atomics and is deterministic.
+ *   - msda_backward_det_* are the bit-reproducible backward (what torch.use_deterministic_algorithms(True) selects in
+ *     the Python shim): grad_value is accumulated as 64-bit fixed point, so it is bit-identical across runs, kernel
+ *     selections (tiled / generic, SPLIT, TMA, knobs) and GPUs.  See DESIGN.md section 11.
  */
 #ifndef MSDA_B200_H_
 #define MSDA_B200_H_
@@ -43,7 +47,7 @@
 extern "C" {
 #endif
 
-#define MSDA_ABI_VERSION 2   /* 2: round-2 entry points (knobs, CondInst head, geometry, W-stationary GEMM) */
+#define MSDA_ABI_VERSION 3   /* 2: round-2 entry points (knobs, CondInst head, geometry, W-stationary GEMM); 3: deterministic backward */
 
 #define MSDA_E_BADARG   (-1)   /* null pointer, non-positive dimension, unknown knob                  */
 #define MSDA_E_TOOLARGE (-2)   /* a dimension product exceeds what the kernels index (see msda_b200.h) */
@@ -130,6 +134,29 @@ int msda_backward_bf16(const uint16_t *grad_out, const uint16_t *value,
                        float *grad_value_f32, uint16_t *grad_value,
                        float *grad_sampling_loc, float *grad_attn_weight, void *stream);
 
+/* ---- deterministic backward: same arguments and results as msda_backward_f32 / _bf16, bit-reproducible grad_value ----
+ * `acc` is caller-allocated int64 scratch of MSDA_DET_HEADER_WORDS + N*S*M*D words, 8-byte aligned (zero-filled by the
+ * callee); its header holds max|attn_weight|, max|grad_out| and a non-finite flag, the rest the fixed-point sums.  grad_value
+ * (fp32) / grad_value_f32 (bf16) must not alias it.  For bf16, grad_value_f32 is scratch for non-finite contributions and
+ * receives the fp32 result only when grad_value == NULL.  No host synchronisation: capture-safe.
+ * Every contribution fp32(fp32(corner_weight * attn) * grad_out) is rounded to the nearest multiple of a power-of-two quantum
+ * 2^(e + ceil(log2(Lq*L*P)) - 62), with 2^e >= max|attn| * max|grad_out|, and summed exactly; NaN / +-Inf contributions are
+ * summed in IEEE fp32 apart (order-independent) and added at the end.  The kernel-selection knobs SLAB, F32_VEC8_BWD and
+ * BF16_FINE_ROWS do not apply here; the tiled kernels (linear / TMA / SPLIT) and the generic kernel are chosen as in the
+ * default path and give identical bits.  There is no deterministic fp64 backward. */
+#define MSDA_DET_HEADER_WORDS 4
+int msda_backward_det_f32(const float *grad_out, const float *value,
+                          const int64_t *spatial_shapes, const int64_t *level_start_index,
+                          const float *sampling_loc, const float *attn_weight,
+                          int N, int S, int M, int D, int L, int Lq, int P,
+                          int64_t *acc, float *grad_value, float *grad_sampling_loc, float *grad_attn_weight, void *stream);
+int msda_backward_det_bf16(const uint16_t *grad_out, const uint16_t *value,
+                           const int64_t *spatial_shapes, const int64_t *level_start_index,
+                           const float *sampling_loc, const float *attn_weight,
+                           int N, int S, int M, int D, int L, int Lq, int P,
+                           int64_t *acc, float *grad_value_f32, uint16_t *grad_value,
+                           float *grad_sampling_loc, float *grad_attn_weight, void *stream);
+
 /* ---- callers of the op (SURVEY.md section 8 rows f-1 / f-2): one-pass fp32 kernels around the cuBLAS GEMMs --------
  * msda_prologue_forward_f32: raw projection -> attention softmax + sampling locations in the op's layouts.
  *   Replaces the five elementwise passes of ops/modules/ms_deform_attn.py:99-112.
@@ -152,6 +179,19 @@ int msda_colsum_f32(const float *x, int64_t rows, int cols, float *out, void *st
 /* ReLU backward fused with the bias gradient of the Linear before it (FFN linear1): g2 = g where y > 0 else 0;
  * colsum[c] = sum_r g2[r, c] (zero-filled by the callee).  cols % 4 == 0. */
 int msda_relu_backward_colsum_f32(const float *g, const float *y, int64_t rows, int cols, float *g2, float *colsum, void *stream);
+/* Deterministic variants (no float atomics; what torch.use_deterministic_algorithms(True) selects in the Python wrappers):
+ * each CTA writes its partial row, summed in a fixed order, to caller-allocated `scratch`, and a second kernel adds the rows
+ * in index order.  The grid depends only on (rows, cols), so results are bit-identical across runs and GPUs.  Scratch
+ * sizes come from the host-only query functions (0 and *bytes on success, MSDA_E_BADARG on bad arguments); scratch must be
+ * 16-byte aligned.  The results are fully written (no zero-fill needed). */
+int msda_colsum_det_scratch_bytes(int64_t rows, int cols, int64_t *bytes);    /* colsum and relu_backward_colsum */
+int msda_layernorm_backward_det_scratch_bytes(int64_t rows, int cols, int64_t *bytes);
+int msda_colsum_det_f32(const float *x, int64_t rows, int cols, float *scratch, float *out, void *stream);
+int msda_relu_backward_colsum_det_f32(const float *g, const float *y, int64_t rows, int cols, float *g2, float *scratch,
+                                      float *colsum, void *stream);
+int msda_layernorm_backward_det_f32(const float *dy, const float *z, const float *gamma, const float *mean,
+                                    const float *rstd, int64_t rows, int cols, float *dz, float *scratch, float *dgamma,
+                                    float *dbeta, void *stream);
 int msda_add_layernorm_forward_f32(const float *a, const float *b, const float *gamma, const float *beta,
                                    int64_t rows, int cols, float eps, float *z, float *y, float *mean, float *rstd,
                                    void *stream);
@@ -187,7 +227,8 @@ int msda_sine_pos_embed_backward_f32(const float *pos, const float *grad_out, in
  *     stride = mask_feat_stride; rel_coord = 1 prepends (ref - pixel location) as two input channels, 0 feeds zeros;
  *     logits [I, H, W].
  * msda_condinst_backward_f32: grad_feats [N, 8, H, W], grad_params [I, 169] and grad_refs [I, 2] (all zero-filled by the
- *   callee, then accumulated with fp32 reductions: summation order, hence the last bits, vary from run to run).
+ *   callee, then accumulated with fp32 reductions: summation order, hence the last bits, vary from run to run;
+ *   msda_condinst_backward_det_f32 below is the bit-reproducible variant).
  * msda_aligned_bilinear_forward/backward_f32: `aligned_bilinear` (ddetrs.py:921-942) on [planes, h, w] -> [planes, f*h, f*w]. */
 int msda_condinst_forward_f32(const float *feats, const float *params, const float *refs, const int32_t *inst_start,
                               int N, int H, int W, int I, int max_inst, int stride, int rel_coord, float *logits,
@@ -195,6 +236,14 @@ int msda_condinst_forward_f32(const float *feats, const float *params, const flo
 int msda_condinst_backward_f32(const float *grad_logits, const float *feats, const float *params, const float *refs,
                                const int32_t *inst_start, int N, int H, int W, int I, int max_inst, int stride,
                                int rel_coord, float *grad_feats, float *grad_params, float *grad_refs, void *stream);
+/* Deterministic CondInst backward: same arguments and results as msda_condinst_backward_f32 plus caller scratch of
+ * msda_condinst_backward_det_scratch_bytes() bytes (per-instance-chunk feature partials and per-warp parameter partials,
+ * added in a fixed order by a second kernel); no float atomics, bit-identical across runs and GPUs. */
+int msda_condinst_backward_det_scratch_bytes(int N, int H, int W, int I, int max_inst, int64_t *bytes);
+int msda_condinst_backward_det_f32(const float *grad_logits, const float *feats, const float *params, const float *refs,
+                                   const int32_t *inst_start, int N, int H, int W, int I, int max_inst, int stride,
+                                   int rel_coord, float *scratch, float *grad_feats, float *grad_params, float *grad_refs,
+                                   void *stream);
 int msda_aligned_bilinear_forward_f32(const float *in, int64_t planes, int h, int w, int factor, float *out, void *stream);
 int msda_aligned_bilinear_backward_f32(const float *grad_out, int64_t planes, int h, int w, int factor, float *grad_in,
                                        void *stream);

@@ -28,10 +28,17 @@ SIGNATURES = {
     "msda_backward_f32": (_i, [_vp] * 6 + _DIMS + [_vp] * 3 + [_vp]),
     "msda_backward_f64": (_i, [_vp] * 6 + _DIMS + [_vp] * 3 + [_vp]),
     "msda_backward_bf16": (_i, [_vp] * 6 + _DIMS + [_vp] * 4 + [_vp]),
+    "msda_backward_det_f32": (_i, [_vp] * 6 + _DIMS + [_vp] * 4 + [_vp]),
+    "msda_backward_det_bf16": (_i, [_vp] * 6 + _DIMS + [_vp] * 5 + [_vp]),
     "msda_prologue_forward_f32": (_i, [_vp] * 3 + [ctypes.c_int64, _i, _i, _i, _i] + [_vp] * 3),
     "msda_prologue_backward_f32": (_i, [_vp] * 5 + [ctypes.c_int64, _i, _i, _i, _i] + [_vp] * 2),
     "msda_colsum_f32": (_i, [_vp, ctypes.c_int64, _i, _vp, _vp]),
     "msda_relu_backward_colsum_f32": (_i, [_vp, _vp, ctypes.c_int64, _i, _vp, _vp, _vp]),
+    "msda_colsum_det_scratch_bytes": (_i, [ctypes.c_int64, _i, _vp]),
+    "msda_layernorm_backward_det_scratch_bytes": (_i, [ctypes.c_int64, _i, _vp]),
+    "msda_colsum_det_f32": (_i, [_vp, ctypes.c_int64, _i, _vp, _vp, _vp]),
+    "msda_relu_backward_colsum_det_f32": (_i, [_vp, _vp, ctypes.c_int64, _i, _vp, _vp, _vp, _vp]),
+    "msda_layernorm_backward_det_f32": (_i, [_vp] * 5 + [ctypes.c_int64, _i] + [_vp] * 5),
     "msda_add_layernorm_forward_f32": (_i, [_vp] * 4 + [ctypes.c_int64, _i, ctypes.c_float] + [_vp] * 5),
     "msda_layernorm_backward_f32": (_i, [_vp] * 5 + [ctypes.c_int64, _i] + [_vp] * 4),
     "msda_linear_tf32": (_i, [_vp] * 3 + [ctypes.c_int64, _i, _i, _vp, _vp]),
@@ -44,15 +51,25 @@ SIGNATURES = {
     "msda_sine_pos_embed_backward_f32": (_i, [_vp, _vp, ctypes.c_int64, _i, _i, ctypes.c_float, _i, _vp, _vp]),
     "msda_condinst_forward_f32": (_i, [_vp] * 4 + [_i] * 7 + [_vp, _vp]),
     "msda_condinst_backward_f32": (_i, [_vp] * 5 + [_i] * 7 + [_vp] * 4),
+    "msda_condinst_backward_det_scratch_bytes": (_i, [_i] * 5 + [_vp]),
+    "msda_condinst_backward_det_f32": (_i, [_vp] * 5 + [_i] * 7 + [_vp] * 5),
     "msda_aligned_bilinear_forward_f32": (_i, [_vp, ctypes.c_int64, _i, _i, _i, _vp, _vp]),
     "msda_aligned_bilinear_backward_f32": (_i, [_vp, ctypes.c_int64, _i, _i, _i, _vp, _vp]),
     "msda_debug_gemm_timeline": (_i, [_vp, _i]),
 }
-ABI_VERSION = 2
+ABI_VERSION = 3
+DET_HEADER_WORDS = 4                                                                                  # MSDA_DET_HEADER_WORDS
 (KNOB_SLAB, KNOB_BWD_WIN_ROWS, KNOB_BWD_LIST_CAP, KNOB_FWD_SLAB_CTAS, KNOB_F32_VEC8_FWD, KNOB_F32_VEC8_BWD,
  KNOB_BF16_FINE_ROWS, KNOB_BF16_PACKED_FWD, KNOB_ZERO_FILL) = range(9)                                                      # include/msda_b200.h
 
 _lib = None
+
+
+def scratch_bytes(query, *args) -> int:
+    """Bytes of scratch a deterministic entry point needs, from its host-only query function."""
+    out = ctypes.c_int64(0)
+    check(query(*args, ctypes.byref(out)), query.__name__)
+    return out.value
 
 
 class MSDALibraryError(RuntimeError):

@@ -20,7 +20,7 @@ LIB_PATH = os.path.join(LIB_DIR, "libmsda_b200.so")
 INCLUDE = os.path.join(os.path.dirname(PKG_DIR), "include")
 
 SOURCES = ["msda_cabi.cu", "msda_gemm_sm100.cu"]
-HEADERS = ["msda_common.cuh", "msda_tiled.cuh", "msda_slab.cuh", "msda_tmem.cuh", "msda_generic.cuh", "msda_module.cuh", "msda_condinst.cuh"]
+HEADERS = ["msda_common.cuh", "msda_tiled.cuh", "msda_slab.cuh", "msda_tmem.cuh", "msda_generic.cuh", "msda_det.cuh", "msda_module.cuh", "msda_condinst.cuh"]
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",

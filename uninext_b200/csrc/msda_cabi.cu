@@ -207,22 +207,23 @@ cudaError_t launch_fwd(const T *value, const int64_t *shapes, const int64_t *lsi
     return cudaGetLastError();
 }
 
-template <typename T, int D, int LP_MAX, int VEC = BwdVec<T>::v>
+template <typename T, int D, int LP_MAX, int VEC = BwdVec<T>::v, bool DET = false>
 cudaError_t launch_bwd(const T *grad_out, const T *value, const int64_t *shapes, const int64_t *lsi, const float *loc,
-                       const float *attn, const Dims &d, float *gv, float *gl, float *ga, cudaStream_t st) {
+                       const float *attn, const Dims &d, float *gv, float *gl, float *ga, cudaStream_t st,
+                       unsigned long long *det_acc, int det_clog2) {
     constexpr int GPW = 32 / (D / VEC);
     constexpr bool kCanStage = (LP_MAX <= 16);
     constexpr bool kCanSplit = (LP_MAX % GPW == 0) && (LP_MAX / GPW <= D / VEC);
     const unsigned npairs = (unsigned)((long long)d.N * d.Lq * d.M);
     const bool split = kCanSplit && use_split(npairs);
     const bool tma = !split && kCanStage && use_tma_staging(d);
-    auto kern = split ? msda::msda_bwd_tiled<T, VEC, D, LP_MAX, kBwdMinCtas, false, kCanSplit>
-                : tma ? msda::msda_bwd_tiled<T, VEC, D, LP_MAX, kBwdMinCtas, kCanStage, false>
-                      : msda::msda_bwd_tiled<T, VEC, D, LP_MAX, kBwdMinCtas, false, false>;
+    auto kern = split ? msda::msda_bwd_tiled<T, VEC, D, LP_MAX, kBwdMinCtas, false, kCanSplit, false, DET>
+                : tma ? msda::msda_bwd_tiled<T, VEC, D, LP_MAX, kBwdMinCtas, kCanStage, false, false, DET>
+                      : msda::msda_bwd_tiled<T, VEC, D, LP_MAX, kBwdMinCtas, false, false, false, DET>;
     static std::atomic<int> c_split[kMaxDevices], c_tma[kMaxDevices], c_ldg[kMaxDevices];
-    const int slots = split ? resident_ctas_cached(msda::msda_bwd_tiled<T, VEC, D, LP_MAX, kBwdMinCtas, false, kCanSplit>, c_split)
-                      : tma ? resident_ctas_cached(msda::msda_bwd_tiled<T, VEC, D, LP_MAX, kBwdMinCtas, kCanStage, false>, c_tma)
-                            : resident_ctas_cached(msda::msda_bwd_tiled<T, VEC, D, LP_MAX, kBwdMinCtas, false, false>, c_ldg);
+    const int slots = split ? resident_ctas_cached(msda::msda_bwd_tiled<T, VEC, D, LP_MAX, kBwdMinCtas, false, kCanSplit, false, DET>, c_split)
+                      : tma ? resident_ctas_cached(msda::msda_bwd_tiled<T, VEC, D, LP_MAX, kBwdMinCtas, kCanStage, false, false, DET>, c_tma)
+                            : resident_ctas_cached(msda::msda_bwd_tiled<T, VEC, D, LP_MAX, kBwdMinCtas, false, false, false, DET>, c_ldg);
     const unsigned iter_pairs = msda::kTiledWarps * (split ? 1 : GPW);
     const unsigned tiles_ub = (npairs + iter_pairs - 1) / iter_pairs;
     const int grid = (int)(tiles_ub < (unsigned)slots ? tiles_ub : (unsigned)slots);
@@ -240,12 +241,13 @@ cudaError_t launch_bwd(const T *grad_out, const T *value, const int64_t *shapes,
         cfg.attrs = attr;
         cfg.numAttrs = 1;
         const cudaError_t e = cudaLaunchKernelEx(&cfg, kern, grad_out, value, shapes, lsi, loc, attn, d.N, d.S, d.M, d.L, d.Lq,
-                                                 d.P, npairs, allow_patches(), gv, gl, ga, (__nv_bfloat16 *)nullptr, 0);
+                                                 d.P, npairs, allow_patches(), gv, gl, ga, (__nv_bfloat16 *)nullptr, 0,
+                                                 det_acc, det_clog2);
         g_launches.fetch_add(1, std::memory_order_relaxed);
         return e != cudaSuccess ? e : cudaGetLastError();
     }
     kern<<<grid, msda::kTiledThreads, 0, st>>>(grad_out, value, shapes, lsi, loc, attn, d.N, d.S, d.M, d.L, d.Lq, d.P,
-                                               npairs, allow_patches(), gv, gl, ga, nullptr, 0);
+                                               npairs, allow_patches(), gv, gl, ga, nullptr, 0, det_acc, det_clog2);
     g_launches.fetch_add(1, std::memory_order_relaxed);
     return cudaGetLastError();
 }
@@ -334,7 +336,7 @@ cudaError_t launch_bwd_mixed(const __nv_bfloat16 *go, const __nv_bfloat16 *value
     const int grid = (int)(tiles_ub < (unsigned)slots ? tiles_ub : (unsigned)slots);
     (tma ? k_tma : k_ldg)<<<grid, msda::kTiledThreads, 0, st>>>(go, value, shapes, lsi, loc, attn, d.N, d.S, d.M, d.L, d.Lq,
                                                                  d.P, npairs, allow_patches(), scratch, gl, ga, gv16,
-                                                                 fine_min_rows);
+                                                                 fine_min_rows, nullptr, 0);
     g_launches.fetch_add(1, std::memory_order_relaxed);
     return cudaGetLastError();
 }
@@ -399,12 +401,12 @@ cudaError_t bwd_fast(const T *go, const T *value, const int64_t *shapes, const i
     if constexpr (sizeof(T) == 4) {
         if (knob(MSDA_KNOB_F32_VEC8_BWD) == 1 && LP <= 16 && d.D == 32 &&
             !((reinterpret_cast<uintptr_t>(value) | reinterpret_cast<uintptr_t>(go)) & 31u))
-            return launch_bwd<T, 32, 16, 8>(go, value, shapes, lsi, loc, attn, d, gv, gl, ga, st);
+            return launch_bwd<T, 32, 16, 8>(go, value, shapes, lsi, loc, attn, d, gv, gl, ga, st, nullptr, 0);
     }
     switch (d.D) {
-        case 16: if constexpr (sizeof(T) == 4) return MSDA_ROUTE_LP(T, 16, launch_bwd)(go, value, shapes, lsi, loc, attn, d, gv, gl, ga, st); break;
-        case 32: return MSDA_ROUTE_LP(T, 32, launch_bwd)(go, value, shapes, lsi, loc, attn, d, gv, gl, ga, st);
-        case 64: return MSDA_ROUTE_LP(T, 64, launch_bwd)(go, value, shapes, lsi, loc, attn, d, gv, gl, ga, st);
+        case 16: if constexpr (sizeof(T) == 4) return MSDA_ROUTE_LP(T, 16, launch_bwd)(go, value, shapes, lsi, loc, attn, d, gv, gl, ga, st, nullptr, 0); break;
+        case 32: return MSDA_ROUTE_LP(T, 32, launch_bwd)(go, value, shapes, lsi, loc, attn, d, gv, gl, ga, st, nullptr, 0);
+        case 64: return MSDA_ROUTE_LP(T, 64, launch_bwd)(go, value, shapes, lsi, loc, attn, d, gv, gl, ga, st, nullptr, 0);
     }
     return cudaErrorInvalidValue;
 }
@@ -422,17 +424,69 @@ cudaError_t fwd_generic(const T *value, const int64_t *shapes, const int64_t *ls
     return cudaGetLastError();
 }
 
-template <typename T, typename TL, typename GA>
+template <typename T, typename TL, typename GA, bool DET = false>
 cudaError_t bwd_generic(const T *go, const T *value, const int64_t *shapes, const int64_t *lsi, const TL *loc,
-                        const TL *attn, const Dims &d, GA *gv, TL *gl, TL *ga, cudaStream_t st) {
+                        const TL *attn, const Dims &d, GA *gv, TL *gl, TL *ga, cudaStream_t st,
+                        unsigned long long *det_acc = nullptr, int det_clog2 = 0) {
     const long long npairs = (long long)d.N * d.Lq * d.M;
     int threads = ((d.D + 31) / 32) * 32;
     if (threads > 256) threads = 256;
     long long blocks = npairs;
     const long long cap = (long long)num_sms() * 64;
     if (blocks > cap) blocks = cap;
-    msda::msda_bwd_generic<T, TL, GA><<<(int)blocks, threads, 0, st>>>(go, value, shapes, lsi, loc, attn, d.S, d.M, d.D,
-                                                                       d.L, d.Lq, d.P, npairs, gv, gl, ga);
+    msda::msda_bwd_generic<T, TL, GA, DET><<<(int)blocks, threads, 0, st>>>(go, value, shapes, lsi, loc, attn, d.S, d.M,
+                                                                            d.D, d.L, d.Lq, d.P, npairs, gv, gl, ga,
+                                                                            det_acc, det_clog2);
+    g_launches.fetch_add(1, std::memory_order_relaxed);
+    return cudaGetLastError();
+}
+
+// ---- deterministic backward (msda_det.cuh) -------------------------------------------------------------------------
+// Tiled kernels (linear / TMA / SPLIT, chosen as in the default path) or the generic kernel accumulate into the
+// fixed-point sums; the slab / tensor-memory kernels, VEC8 lanes and BF16_FINE_ROWS do not apply.
+static_assert(msda::kDetHeaderWords == MSDA_DET_HEADER_WORDS, "accumulator header size");
+
+template <typename T>
+cudaError_t bwd_det(const T *go, const T *value, const int64_t *shapes, const int64_t *lsi, const float *loc,
+                    const float *attn, const Dims &d, bool aligned, int64_t *acc, float *nf, float *gl, float *ga,
+                    float *out32, __nv_bfloat16 *out16, cudaStream_t st) {
+    unsigned long long *hdr = reinterpret_cast<unsigned long long *>(acc);
+    const long long nval = (long long)d.N * d.S * d.M * d.D;
+    int clog2 = 0;                                       // K = Lq * L * P contributions per row at most
+    while ((1ll << clog2) < (long long)d.Lq * d.L * d.P) ++clog2;
+    cudaError_t err = zero_fill(acc, sizeof(int64_t) * (size_t)(nval + msda::kDetHeaderWords), st);
+    if (err != cudaSuccess) return err;
+    const int wave = num_sms() * 4;
+    msda::msda_det_scale<T><<<wave, 256, 0, st>>>(attn, (long long)d.N * d.Lq * d.M * d.L * d.P, go,
+                                                  (long long)d.N * d.Lq * d.M * d.D, hdr);
+    msda::msda_det_prepare<<<wave, 256, 0, st>>>(hdr, clog2, nf, nval);
+    g_launches.fetch_add(2, std::memory_order_relaxed);
+    if ((err = cudaGetLastError()) != cudaSuccess) return err;
+    const int LP = d.L * d.P;
+    if (aligned && use_fast(sizeof(T), d)) {
+        switch (d.D) {
+            case 16:
+                if constexpr (sizeof(T) == 4) {
+                    err = LP <= 16 ? launch_bwd<T, 16, 16, 4, true>(go, value, shapes, lsi, loc, attn, d, nf, gl, ga, st, hdr, clog2)
+                                   : launch_bwd<T, 16, 32, 4, true>(go, value, shapes, lsi, loc, attn, d, nf, gl, ga, st, hdr, clog2);
+                }
+                break;
+            case 32:
+                err = LP <= 16 ? launch_bwd<T, 32, 16, 4, true>(go, value, shapes, lsi, loc, attn, d, nf, gl, ga, st, hdr, clog2)
+                               : launch_bwd<T, 32, 32, 4, true>(go, value, shapes, lsi, loc, attn, d, nf, gl, ga, st, hdr, clog2);
+                break;
+            case 64:
+                err = LP <= 16 ? launch_bwd<T, 64, 16, 4, true>(go, value, shapes, lsi, loc, attn, d, nf, gl, ga, st, hdr, clog2)
+                               : launch_bwd<T, 64, 32, 4, true>(go, value, shapes, lsi, loc, attn, d, nf, gl, ga, st, hdr, clog2);
+                break;
+        }
+    } else {
+        err = bwd_generic<T, float, float, true>(go, value, shapes, lsi, loc, attn, d, nf, gl, ga, st, hdr, clog2);
+    }
+    if (err != cudaSuccess) return err;
+    long long blocks = (nval + 255) / 256;
+    if (blocks > (long long)num_sms() * 16) blocks = (long long)num_sms() * 16;
+    msda::msda_det_convert<<<(int)blocks, 256, 0, st>>>(hdr, clog2, nf, nval, out32, out16);
     g_launches.fetch_add(1, std::memory_order_relaxed);
     return cudaGetLastError();
 }
@@ -610,6 +664,34 @@ int msda_backward_bf16(const uint16_t *grad_out, const uint16_t *value, const in
     return (int)err;
 }
 
+int msda_backward_det_f32(const float *grad_out, const float *value, const int64_t *spatial_shapes,
+                          const int64_t *level_start_index, const float *sampling_loc, const float *attn_weight, int N,
+                          int S, int M, int D, int L, int Lq, int P, int64_t *acc, float *grad_value,
+                          float *grad_sampling_loc, float *grad_attn_weight, void *stream) {
+    const Dims d{N, S, M, D, L, Lq, P};
+    if (int e = check_dims(d)) return e;
+    MSDA_CHECK_PTRS(al, grad_out, value, sampling_loc, attn_weight, grad_value, grad_sampling_loc, grad_attn_weight);
+    if (!spatial_shapes || !level_start_index || !acc || (reinterpret_cast<uintptr_t>(acc) & 7u)) return MSDA_E_BADARG;
+    return (int)bwd_det<float>(grad_out, value, spatial_shapes, level_start_index, sampling_loc, attn_weight, d, al, acc,
+                               grad_value, grad_sampling_loc, grad_attn_weight, grad_value, nullptr,
+                               static_cast<cudaStream_t>(stream));
+}
+
+int msda_backward_det_bf16(const uint16_t *grad_out, const uint16_t *value, const int64_t *spatial_shapes,
+                           const int64_t *level_start_index, const float *sampling_loc, const float *attn_weight, int N,
+                           int S, int M, int D, int L, int Lq, int P, int64_t *acc, float *grad_value_f32,
+                           uint16_t *grad_value, float *grad_sampling_loc, float *grad_attn_weight, void *stream) {
+    const Dims d{N, S, M, D, L, Lq, P};
+    if (int e = check_dims(d)) return e;
+    MSDA_CHECK_PTRS(al, grad_out, value, sampling_loc, attn_weight, grad_value_f32, grad_sampling_loc, grad_attn_weight);
+    if (!spatial_shapes || !level_start_index || !acc || (reinterpret_cast<uintptr_t>(acc) & 7u)) return MSDA_E_BADARG;
+    __nv_bfloat16 *gv16 = reinterpret_cast<__nv_bfloat16 *>(grad_value);
+    return (int)bwd_det<__nv_bfloat16>(reinterpret_cast<const __nv_bfloat16 *>(grad_out),
+                                       reinterpret_cast<const __nv_bfloat16 *>(value), spatial_shapes, level_start_index,
+                                       sampling_loc, attn_weight, d, al, acc, grad_value_f32, grad_sampling_loc,
+                                       grad_attn_weight, gv16 ? nullptr : grad_value_f32, gv16,
+                                       static_cast<cudaStream_t>(stream));
+}
 
 }  // extern "C"
 
@@ -697,6 +779,90 @@ int msda_relu_backward_colsum_f32(const float *g, const float *y, int64_t rows, 
     return (int)cudaGetLastError();
 }
 
+}  // extern "C"
+
+// ---- deterministic caller reductions: partial rows per CTA in caller scratch, then a fixed-order sum ---------------------
+// The grid is a function of (rows, cols) only -- at most kDetParts CTAs -- so the result is bit-identical on any GPU and the
+// scratch size is known on the host.
+namespace {
+constexpr long long kDetParts = 512;
+long long det_rows_per_cta(long long rows, int multiple) {
+    long long r = (rows + kDetParts - 1) / kDetParts;
+    if (r < 16) r = 16;
+    return (r + multiple - 1) / multiple * multiple;
+}
+long long det_parts(long long rows, int multiple) {
+    const long long r = det_rows_per_cta(rows, multiple);
+    return (rows + r - 1) / r;
+}
+bool ln_cols_ok(int cols) { return cols == 128 || cols == 256 || cols == 384 || cols == 512; }
+cudaError_t sum_partials(const float *part, long long nparts, int cols, float *out, cudaStream_t st) {
+    msda::msda_sum_partials<<<(cols + 255) / 256, 256, 0, st>>>(part, (int)nparts, cols, out);
+    g_launches.fetch_add(1, std::memory_order_relaxed);
+    return cudaGetLastError();
+}
+}  // namespace
+
+extern "C" {
+
+int msda_colsum_det_scratch_bytes(int64_t rows, int cols, int64_t *bytes) {
+    if (!bytes || rows <= 0 || cols <= 0 || cols % 4 != 0) return MSDA_E_BADARG;
+    *bytes = (int64_t)(det_parts(rows, 1) * cols * (long long)sizeof(float));
+    return 0;
+}
+
+int msda_layernorm_backward_det_scratch_bytes(int64_t rows, int cols, int64_t *bytes) {
+    if (!bytes || rows <= 0 || !ln_cols_ok(cols)) return MSDA_E_BADARG;
+    *bytes = (int64_t)(2 * det_parts(rows, 8) * cols * (long long)sizeof(float));
+    return 0;
+}
+
+int msda_colsum_det_f32(const float *x, int64_t rows, int cols, float *scratch, float *out, void *stream) {
+    if (!x || !out || !scratch || rows <= 0 || cols <= 0 || cols % 4 != 0 || !aligned16(x) || !aligned16(scratch))
+        return MSDA_E_BADARG;
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    const long long rpc = det_rows_per_cta(rows, 1), parts = det_parts(rows, 1);
+    msda::msda_colsum<true><<<(unsigned)parts, 256, 0, st>>>(x, rows, cols, (int)rpc, scratch);
+    g_launches.fetch_add(1, std::memory_order_relaxed);
+    const cudaError_t err = cudaGetLastError();
+    return (int)(err != cudaSuccess ? err : sum_partials(scratch, parts, cols, out, st));
+}
+
+int msda_relu_backward_colsum_det_f32(const float *g, const float *y, int64_t rows, int cols, float *g2, float *scratch,
+                                      float *colsum, void *stream) {
+    if (!g || !y || !g2 || !scratch || !colsum || rows <= 0 || cols <= 0 || cols % 4 != 0 || !aligned16(g) || !aligned16(y) ||
+        !aligned16(g2) || !aligned16(scratch))
+        return MSDA_E_BADARG;
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    const long long rpc = det_rows_per_cta(rows, 1), parts = det_parts(rows, 1);
+    msda::msda_relu_bwd_colsum<true><<<(unsigned)parts, 256, 0, st>>>(g, y, rows, cols, (int)rpc, g2, scratch);
+    g_launches.fetch_add(1, std::memory_order_relaxed);
+    const cudaError_t err = cudaGetLastError();
+    return (int)(err != cudaSuccess ? err : sum_partials(scratch, parts, cols, colsum, st));
+}
+
+int msda_layernorm_backward_det_f32(const float *dy, const float *z, const float *gamma, const float *mean, const float *rstd,
+                                    int64_t rows, int cols, float *dz, float *scratch, float *dgamma, float *dbeta,
+                                    void *stream) {
+    if (!dy || !z || !gamma || !mean || !rstd || !dz || !scratch || !dgamma || !dbeta || rows <= 0 || !ln_cols_ok(cols))
+        return MSDA_E_BADARG;
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    const long long rpc = det_rows_per_cta(rows, 8), parts = det_parts(rows, 8);
+    float *pg = scratch, *pb = scratch + parts * cols;
+    const unsigned grid = (unsigned)parts;
+    switch (cols / 128) {
+        case 1: msda::msda_layernorm_bwd<1, true><<<grid, 256, 0, st>>>(dy, z, gamma, mean, rstd, rows, (int)rpc, dz, pg, pb); break;
+        case 2: msda::msda_layernorm_bwd<2, true><<<grid, 256, 0, st>>>(dy, z, gamma, mean, rstd, rows, (int)rpc, dz, pg, pb); break;
+        case 3: msda::msda_layernorm_bwd<3, true><<<grid, 256, 0, st>>>(dy, z, gamma, mean, rstd, rows, (int)rpc, dz, pg, pb); break;
+        default: msda::msda_layernorm_bwd<4, true><<<grid, 256, 0, st>>>(dy, z, gamma, mean, rstd, rows, (int)rpc, dz, pg, pb); break;
+    }
+    g_launches.fetch_add(1, std::memory_order_relaxed);
+    cudaError_t err = cudaGetLastError();
+    if (err == cudaSuccess) err = sum_partials(pg, parts, cols, dgamma, st);
+    if (err == cudaSuccess) err = sum_partials(pb, parts, cols, dbeta, st);
+    return (int)err;
+}
+
 int msda_add_layernorm_forward_f32(const float *a, const float *b, const float *gamma, const float *beta, int64_t rows,
                                    int cols, float eps, float *z, float *y, float *mean, float *rstd, void *stream) {
     if (!a || !gamma || !beta || !y || !mean || !rstd || rows <= 0 || (b != nullptr && z == nullptr)) return MSDA_E_BADARG;
@@ -771,6 +937,41 @@ int msda_condinst_backward_f32(const float *grad_logits, const float *feats, con
     msda::condinst_bwd<<<grid, msda::kCiThreads, 0, st>>>(grad_logits, feats, params, refs, inst_start, HW, W, stride, rel_coord,
                                                           grad_feats, grad_params, grad_refs);
     g_launches.fetch_add(1, std::memory_order_relaxed);
+    return (int)cudaGetLastError();
+}
+
+// Partials of the deterministic CondInst backward: [ceil(max_inst / 16)][N][8][H*W] feature partials, then
+// [ceil(H*W / 64)][I][171] per-warp sums.
+int msda_condinst_backward_det_scratch_bytes(int N, int H, int W, int I, int max_inst, int64_t *bytes) {
+    if (!bytes || N <= 0 || H <= 0 || W <= 0 || I < 0 || max_inst < 0 || (long long)H * W >= (1ll << 30)) return MSDA_E_BADARG;
+    const long long HW = (long long)H * W, chunks = (max_inst + msda::kCiChunk - 1) / msda::kCiChunk;
+    *bytes = (int64_t)(sizeof(float) * (chunks * N * msda::kCiFeat * HW + ((HW + 63) / 64) * (long long)I * msda::kCiSums));
+    return 0;
+}
+
+int msda_condinst_backward_det_f32(const float *grad_logits, const float *feats, const float *params, const float *refs,
+                                   const int32_t *inst_start, int N, int H, int W, int I, int max_inst, int stride,
+                                   int rel_coord, float *scratch, float *grad_feats, float *grad_params, float *grad_refs,
+                                   void *stream) {
+    if (!grad_logits || !feats || !params || !refs || !inst_start || !scratch || !grad_feats || !grad_params || !grad_refs ||
+        N <= 0 || H <= 0 || W <= 0 || I < 0 || max_inst < 0 || stride <= 0 || (long long)H * W >= (1ll << 30))
+        return MSDA_E_BADARG;
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    const int HW = H * W, tile = msda::kCiThreads * msda::kCiBwdPpt;
+    if (I == 0 || max_inst == 0)
+        return (int)cudaMemsetAsync(grad_feats, 0, sizeof(float) * (size_t)N * msda::kCiFeat * HW, st);
+    const int chunks = (max_inst + msda::kCiChunk - 1) / msda::kCiChunk;
+    float *feat_part = scratch, *sum_part = scratch + (size_t)chunks * N * msda::kCiFeat * HW;
+    const dim3 grid((unsigned)((HW + tile - 1) / tile), (unsigned)chunks, (unsigned)N);
+    msda::condinst_bwd<true><<<grid, msda::kCiThreads, 0, st>>>(grad_logits, feats, params, refs, inst_start, HW, W, stride,
+                                                                rel_coord, grad_feats, grad_params, grad_refs, feat_part,
+                                                                sum_part, I);
+    const long long total = (long long)N * msda::kCiFeat * HW + (long long)I * msda::kCiSums;
+    long long blocks = (total + 255) / 256;
+    if (blocks > (long long)num_sms() * 16) blocks = (long long)num_sms() * 16;
+    msda::condinst_bwd_reduce<<<(unsigned)blocks, 256, 0, st>>>(feat_part, sum_part, inst_start, N, HW, I, (HW + 63) / 64,
+                                                               grad_feats, grad_params, grad_refs);
+    g_launches.fetch_add(2, std::memory_order_relaxed);
     return (int)cudaGetLastError();
 }
 

@@ -72,6 +72,13 @@ __device__ __forceinline__ TapGeom tap_geometry(float x, float y, int H, int W, 
     return g;
 }
 
+// Masked corner weights of a tap with attention weight a (corner k outside the map or window: 0).
+__device__ __forceinline__ float4 masked_weights(const TapGeom &g, float a) {
+    const float hh = 1.f - g.lh, hw = 1.f - g.lw;
+    return make_float4((g.mask & 1u) ? hh * hw * a : 0.f, (g.mask & 2u) ? hh * g.lw * a : 0.f,
+                       (g.mask & 4u) ? g.lh * hw * a : 0.f, (g.mask & 8u) ? g.lh * g.lw * a : 0.f);
+}
+
 // Vector access to one slice of a value / grad row, widened to fp32 registers.  VEC = elements per lane:
 // fp32: 4 (16 bytes); bf16: 8 (16 bytes, forward) or 4 (8 bytes, backward -- keeps one lane's grad_value slice a
 // contiguous 16-byte fp32 quad so that every red.v4 fills whole sectors).

@@ -245,10 +245,15 @@ __device__ __forceinline__ float warp_transpose_sum16(float (&v)[16], int lane) 
 //   warp reduction, one RED per group from lanes 0-15.
 // grid: (pixel tiles, instance chunks, images).  grad_feats [N, 8, H*W], grad_params [I, 169] and grad_refs [I, 2] must be
 // zero on entry.
+// DET: no atomics.  Each thread stores its chunk's feature gradient to feat_part [chunk][N][8][H*W], and each warp stores its
+// 171 per-instance sums to sum_part [warp slot][I][171] (warp slot = global warp index, 64 pixels each); condinst_bwd_reduce
+// then adds the partials in a fixed order.
+template <bool DET = false>
 __global__ void __launch_bounds__(kCiThreads, 3)
 condinst_bwd(const float *__restrict__ grad_logits, const float *__restrict__ feats, const float *__restrict__ params,
              const float *__restrict__ refs, const int *__restrict__ inst_start, int HW, int W, int stride, int rel_coord,
-             float *__restrict__ grad_feats, float *__restrict__ grad_params, float *__restrict__ grad_refs)
+             float *__restrict__ grad_feats, float *__restrict__ grad_params, float *__restrict__ grad_refs,
+             float *__restrict__ feat_part = nullptr, float *__restrict__ sum_part = nullptr, int I = 0)
 {
     static_assert(kCiBwdPpt == 2, "one pixel pair per thread");
     __shared__ __align__(16) float sp[kCiChunk][kCiRow];
@@ -289,7 +294,10 @@ condinst_bwd(const float *__restrict__ grad_logits, const float *__restrict__ fe
             for (int i = 0; i < 16; ++i) v[i] = f2_lo(sums[i]) + f2_hi(sums[i]);
             const float sum = warp_transpose_sum16(v, lane);
             const int j = dst(lane & 15);
-            if (lane < 16 && j >= 0) {
+            if constexpr (DET) {
+                const size_t slot = (size_t)(blockIdx.x * (kCiThreads / 32) + (threadIdx.x >> 5));
+                if (lane < 16 && j >= 0) sum_part[(slot * I + (i0 + k)) * kCiSums + j] = sum;
+            } else if (lane < 16 && j >= 0) {
                 if (j < kCiParams) atomicAdd(grad_params + (size_t)(i0 + k) * kCiParams + j, sum);
                 else atomicAdd(grad_refs + (size_t)(i0 + k) * 2 + (j - kCiParams), sum);
             }
@@ -350,9 +358,41 @@ condinst_bwd(const float *__restrict__ grad_logits, const float *__restrict__ fe
     }
 #pragma unroll
     for (int c = 0; c < kCiFeat; ++c) {
+        if constexpr (DET) {
+            float *dst = feat_part + (((size_t)blockIdx.y * gridDim.z + b) * kCiFeat + c) * HW;
+            if (live0) dst[pa] = f2_lo(gf[c]);
+            if (live1) dst[pb] = f2_hi(gf[c]);
+            continue;
+        }
         float *dst = grad_feats + ((size_t)b * kCiFeat + c) * HW;
         if (live0) atomicAdd(dst + pa, f2_lo(gf[c]));
         if (live1) atomicAdd(dst + pb, f2_hi(gf[c]));
+    }
+}
+
+// Fixed-order reduction of condinst_bwd<true>'s partials.  Threads [0, N*8*HW) sum the feature partials of the instance
+// chunks image b actually has, in chunk order; threads [N*8*HW, + I*171) sum the per-instance partials over the warp slots
+// in slot order.  Every output element is written.
+__global__ void __launch_bounds__(256)
+condinst_bwd_reduce(const float *__restrict__ feat_part, const float *__restrict__ sum_part, const int *__restrict__ inst_start,
+                    int N, int HW, int I, int nslots, float *__restrict__ grad_feats, float *__restrict__ grad_params,
+                    float *__restrict__ grad_refs)
+{
+    const long long nf = (long long)N * kCiFeat * HW, ns = (long long)I * kCiSums;
+    for (long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x; t < nf + ns; t += (long long)gridDim.x * blockDim.x) {
+        float acc = 0.f;
+        if (t < nf) {
+            const int b = (int)(t / ((long long)kCiFeat * HW));
+            const int chunks = (inst_start[b + 1] - inst_start[b] + kCiChunk - 1) / kCiChunk;
+            for (int y = 0; y < chunks; ++y) acc += feat_part[(size_t)y * nf + t];
+            grad_feats[t] = acc;
+        } else {
+            const long long u = t - nf;
+            for (int sl = 0; sl < nslots; ++sl) acc += sum_part[(size_t)sl * ns + u];
+            const int i = (int)(u / kCiSums), j = (int)(u % kCiSums);
+            if (j < kCiParams) grad_params[(size_t)i * kCiParams + j] = acc;
+            else grad_refs[(size_t)i * 2 + (j - kCiParams)] = acc;
+        }
     }
 }
 

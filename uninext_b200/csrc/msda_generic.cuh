@@ -6,6 +6,7 @@
 #pragma once
 
 #include "msda_common.cuh"
+#include "msda_det.cuh"
 
 namespace msda {
 
@@ -94,16 +95,23 @@ __device__ __forceinline__ C block_sum(C v, C *scratch) {
 
 // One block per (b,q,m) pair, threads stride over channels.  GA is the grad_value accumulator type
 // (T for fp32/fp64, float for bf16 storage).
-template <typename T, typename TL, typename GA>
+// DET (fp32 compute only, msda_det.cuh): grad_value goes to the fixed-point sums in det_acc, from the tiled kernels' tap
+// geometry, skip rule and fp32 products, so both families produce the same bits; grad_value only receives non-finite
+// contributions.
+template <typename T, typename TL, typename GA, bool DET = false>
 __global__ void __launch_bounds__(256)
 msda_bwd_generic(const T *__restrict__ grad_out, const T *__restrict__ value,
                  const int64_t *__restrict__ shapes, const int64_t *__restrict__ lsi,
                  const TL *__restrict__ loc, const TL *__restrict__ attn,
                  int S, int M, int D, int L, int Lq, int P, long long npairs,
-                 GA *__restrict__ grad_value, TL *__restrict__ grad_loc, TL *__restrict__ grad_attn)
+                 GA *__restrict__ grad_value, TL *__restrict__ grad_loc, TL *__restrict__ grad_attn,
+                 unsigned long long *__restrict__ det_acc, int det_clog2)
 {
     using C = typename Num<T>::C;
+    static_assert(!DET || sizeof(C) == 4, "DET: fp32 contributions");
     __shared__ C scratch[8];
+    DetScale ds{};
+    if constexpr (DET) ds = det_scale(det_acc, det_clog2);
     for (long long pair = blockIdx.x; pair < npairs; pair += gridDim.x) {
         const int m = (int)(pair % M);
         const long long b = (pair / M) / Lq;
@@ -116,6 +124,22 @@ msda_bwd_generic(const T *__restrict__ grad_out, const T *__restrict__ value,
                 const long long t = (pair * L + l) * P + p;
                 const C a = (C)attn[t];
                 const GTap<C> g = generic_tap<C>((C)loc[2 * t], (C)loc[2 * t + 1], H, W, start);
+                if constexpr (DET) {
+                    const TapGeom gm = tap_geometry((float)loc[2 * t], (float)loc[2 * t + 1], H, W, (int)start);
+                    const float4 w4 = masked_weights(gm, (float)a);
+                    const float w[4] = {w4.x, w4.y, w4.z, w4.w};
+                    const size_t row[4] = {slab + (size_t)gm.r0 * row_elems, slab + (size_t)(gm.r0 + gm.dw) * row_elems,
+                                           slab + (size_t)gm.r1 * row_elems, slab + (size_t)(gm.r1 + gm.dw) * row_elems};
+                    if (gm.mask) {
+                        for (int c = threadIdx.x; c < D; c += blockDim.x) {
+                            const float go = Num<T>::ld(grad_out + (size_t)pair * D + c);
+#pragma unroll
+                            for (int k = 0; k < 4; ++k)
+                                if (w[k] != 0.f)
+                                    det_add(ds, det_acc + kDetHeaderWords, grad_value, row[k] + c, det_contrib(w[k], go));
+                        }
+                    }
+                }
                 C ga = 0, gx = 0, gy = 0;
                 if (g.inside) {
                     const C hh = (C)1 - g.lh, hw = (C)1 - g.lw;
@@ -129,7 +153,7 @@ msda_bwd_generic(const T *__restrict__ grad_out, const T *__restrict__ value,
                             if (g.r[k] >= 0) {
                                 const size_t o = slab + (size_t)g.r[k] * row_elems + c;
                                 v[k] = Num<T>::ld(value + o);
-                                atomicAdd(grad_value + o, (GA)(cw[k] * a * go));            // cuh:125,134,143,152
+                                if constexpr (!DET) atomicAdd(grad_value + o, (GA)(cw[k] * a * go));   // cuh:125,134,143,152
                             }
                         }
                         ga += go * (cw[0] * v[0] + cw[1] * v[1] + cw[2] * v[2] + cw[3] * v[3]);     // cuh:156

@@ -98,8 +98,28 @@ msda_prologue_bwd(const float *__restrict__ grad_loc, const float *__restrict__ 
     row[2 * (m * LP + j) + 1] = g.y;
 }
 
+// Deterministic variants (DET = true) of the column sums below: the CTA's partial row, already summed in a fixed order,
+// is stored to row blockIdx.x of a [gridDim.x, cols] scratch instead of being added to the result with a float red;
+// msda_sum_partials then adds the rows in index order.
+__device__ __forceinline__ void colsum_out(bool det, float *out, int cols, int c, float4 acc) {
+    if (det) reinterpret_cast<float4 *>(out + (size_t)blockIdx.x * cols)[c] = acc;
+    else red_add_v4(out + 4 * c, acc.x, acc.y, acc.z, acc.w);
+}
+
+// out[c] = sum_p part[p, c] for p = 0 .. nparts-1 in order.
+__global__ void __launch_bounds__(256)
+msda_sum_partials(const float *__restrict__ part, int nparts, int cols, float *__restrict__ out)
+{
+    for (int c = blockIdx.x * blockDim.x + threadIdx.x; c < cols; c += gridDim.x * blockDim.x) {
+        float acc = 0.f;
+        for (int p = 0; p < nparts; ++p) acc += part[(size_t)p * cols + c];
+        out[c] = acc;
+    }
+}
+
 // out[c] += sum over this CTA's rows of x[r, c].  `out` must be zero on entry.  Thread (rl, c) sums the float4 column slice
 // c over rows r0+rl, r0+rl+RL, ...; the RL row-lanes are then combined in shared memory and leave as one 16-byte red.
+template <bool DET = false>
 __global__ void __launch_bounds__(256)
 msda_colsum(const float *__restrict__ x, long long rows, int cols, int rows_per_cta, float *__restrict__ out)
 {
@@ -128,7 +148,7 @@ msda_colsum(const float *__restrict__ x, long long rows, int cols, int rows_per_
                 const float4 t = part[k * cs + ct];
                 acc.x += t.x; acc.y += t.y; acc.z += t.z; acc.w += t.w;
             }
-            red_add_v4(out + 4 * c, acc.x, acc.y, acc.z, acc.w);
+            colsum_out(DET, out, cols, c, acc);
         }
         __syncthreads();
     }
@@ -137,6 +157,7 @@ msda_colsum(const float *__restrict__ x, long long rows, int cols, int rows_per_
 // ReLU backward fused with the bias gradient of the Linear in front of it (FFN linear1, deformable_transformer.py:345-349):
 //   g2[r, c] = y[r, c] > 0 ? g[r, c] : 0 ;   out[c] += sum_r g2[r, c]
 // One pass over g and y instead of threshold_backward followed by a separate column-sum read of g2 (366 MB at cfg2).
+template <bool DET = false>
 __global__ void __launch_bounds__(256)
 msda_relu_bwd_colsum(const float *__restrict__ g, const float *__restrict__ y, long long rows, int cols, int rows_per_cta,
                      float *__restrict__ g2, float *__restrict__ out)
@@ -170,7 +191,7 @@ msda_relu_bwd_colsum(const float *__restrict__ g, const float *__restrict__ y, l
                 const float4 t = part[k * cs + ct];
                 acc.x += t.x; acc.y += t.y; acc.z += t.z; acc.w += t.w;
             }
-            red_add_v4(out + 4 * c, acc.x, acc.y, acc.z, acc.w);
+            colsum_out(DET, out, cols, c, acc);
         }
         __syncthreads();
     }
@@ -329,7 +350,8 @@ msda_add_layernorm_fwd(const float *__restrict__ a, const float *__restrict__ b,
 // dz = rstd * (dy*gamma - mean(dy*gamma) - xhat * mean(dy*gamma*xhat));  dgamma += sum_rows dy*xhat;  dbeta += sum_rows dy.
 // Each warp walks rows warp, warp+W, ...; its per-lane column partials are combined across the CTA's warps in shared
 // memory and leave the CTA as one 16-byte red per lane-slice.  dgamma / dbeta must be zero on entry.
-template <int V>
+// DET: dgamma / dbeta are [gridDim.x, cols] scratch rows instead (see colsum_out).
+template <int V, bool DET = false>
 __global__ void __launch_bounds__(256)
 msda_layernorm_bwd(const float *__restrict__ dy, const float *__restrict__ z, const float *__restrict__ gamma,
                    const float *__restrict__ mean, const float *__restrict__ rstd, long long rows, int rows_per_cta,
@@ -380,8 +402,8 @@ msda_layernorm_bwd(const float *__restrict__ dy, const float *__restrict__ z, co
             tg.x += sg[w][c].x; tg.y += sg[w][c].y; tg.z += sg[w][c].z; tg.w += sg[w][c].w;
             tb.x += sb[w][c].x; tb.y += sb[w][c].y; tb.z += sb[w][c].z; tb.w += sb[w][c].w;
         }
-        red_add_v4(dgamma + 4 * c, tg.x, tg.y, tg.z, tg.w);
-        red_add_v4(dbeta + 4 * c, tb.x, tb.y, tb.z, tb.w);
+        colsum_out(DET, dgamma, C, c, tg);
+        colsum_out(DET, dbeta, C, c, tb);
     }
 }
 

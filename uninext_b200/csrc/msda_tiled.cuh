@@ -27,6 +27,7 @@
 #pragma once
 
 #include "msda_common.cuh"
+#include "msda_det.cuh"
 
 namespace msda {
 
@@ -173,12 +174,6 @@ struct TapStage {                       // per-warp double buffer
     static constexpr int kLoc = GPW * LP_MAX * 8, kAttn = GPW * LP_MAX * 4;
     static constexpr int kBytes = ENABLED ? 2 * (kLoc + kAttn) : 16;
 };
-
-__device__ __forceinline__ float4 masked_weights(const TapGeom &g, float a) {
-    const float hh = 1.f - g.lh, hw = 1.f - g.lw;
-    return make_float4((g.mask & 1u) ? hh * hw * a : 0.f, (g.mask & 2u) ? hh * g.lw * a : 0.f,
-                       (g.mask & 4u) ? g.lh * hw * a : 0.f, (g.mask & 8u) ? g.lh * g.lw * a : 0.f);
-}
 
 // ------------------------------------------------------------------------------------------------------------
 // forward:  out[b,q,m,:] = sum_taps a * bilinear(value_l[b,:,m,:], x, y)            (reference cuh:237-299)
@@ -389,16 +384,22 @@ __device__ __forceinline__ void group_reduce_scatter(float (&part)[LPR][4], int 
 // bytes through the SM's crossbar port, which is what bounds this kernel -- while the coarse levels (hundreds to
 // thousands of contributions per row) keep the fp32 accumulator.  The fine flag travels in bit 31 of the record's row
 // index (rows are < 2^30).
-template <typename T, int VEC, int D, int LP_MAX, int MIN_CTAS, bool TMA, bool SPLIT, bool MIXED = false>
+// DET (msda_det.cuh): grad_value is accumulated as 64-bit fixed point in det_acc (header, then the sums), with the
+// same taps, skip rule and fp32 products (det_contrib) as msda_bwd_generic<DET>; grad_value itself only receives
+// non-finite contributions.  u64 reds have no vector form, so each group first transposes its output gradient: in
+// red k lane `sub` owns channel k * LPR + sub, and the LPR lanes of a group write LPR consecutive words of one row.
+template <typename T, int VEC, int D, int LP_MAX, int MIN_CTAS, bool TMA, bool SPLIT, bool MIXED = false, bool DET = false>
 __global__ void __launch_bounds__(kTiledThreads, MIN_CTAS)
 msda_bwd_tiled(const T *__restrict__ grad_out, const T *__restrict__ value,
                const int64_t *__restrict__ shapes, const int64_t *__restrict__ lsi,
                const float *__restrict__ loc, const float *__restrict__ attn,
                int N, int S, int M, int L, int Lq, int P, unsigned npairs, int allow_patches,
                float *__restrict__ grad_value, float *__restrict__ grad_loc, float *__restrict__ grad_attn,
-               __nv_bfloat16 *__restrict__ grad_value_bf16, int fine_min_rows)
+               __nv_bfloat16 *__restrict__ grad_value_bf16, int fine_min_rows, unsigned long long *__restrict__ det_acc,
+               int det_clog2)
 {
     static_assert(!MIXED || (sizeof(T) == 2 && VEC == 4), "MIXED accumulates bf16 rows with 8-byte packed reds");
+    static_assert(!DET || (!MIXED && VEC == 4), "DET: fp32 contributions, 4 channels per lane");
     constexpr int LPR = D / VEC;
     constexpr int GPW = 32 / LPR;
     constexpr int PPW = SPLIT ? 1 : GPW;                    // see msda_fwd_tiled
@@ -445,6 +446,8 @@ msda_bwd_tiled(const T *__restrict__ grad_out, const T *__restrict__ value,
         __syncwarp();
     }
     pdl_wait_primary();      // grad_value's zero-fill (msda_zero_fill as PDL primary) is complete and visible from here on
+    DetScale ds{};
+    if constexpr (DET) ds = det_scale(det_acc, det_clog2);
 
     for (unsigned tile = blockIdx.x; tile < wm.ntiles; tile += gridDim.x) {
         const TileCtx tc = decode_tile(wm, tile, L, M);
@@ -467,6 +470,19 @@ msda_bwd_tiled(const T *__restrict__ grad_out, const T *__restrict__ value,
 
             float g[VEC];
             RowVec<T, VEC>::load(grad_out + (size_t)pair * D + (size_t)sub * VEC, g);
+            float gt[VEC];                       // DET: gt[k] = g of channel k * LPR + sub
+            if constexpr (DET) {
+#pragma unroll
+                for (int k = 0; k < VEC; ++k) {
+                    const int ch = k * LPR + sub;
+                    gt[k] = 0.f;
+#pragma unroll
+                    for (int e = 0; e < VEC; ++e) {
+                        const float t = __shfl_sync(kFullMask, g[e], ch / VEC, LPR);
+                        if (e == ch % VEC) gt[k] = t;
+                    }
+                }
+            }
 
             // ---- stage 1 ----
             float4 tw[NSL];
@@ -527,7 +543,15 @@ msda_bwd_tiled(const T *__restrict__ grad_out, const T *__restrict__ value,
 #pragma unroll
                         for (int e = 0; e < VEC; ++e) dsum = fmaf(g[e], v[e], dsum);
                         part[j][c] = dsum;
-                        if constexpr (MIXED) {        // predicated, branch-free: bf16 result row or fp32 scratch row
+                        if constexpr (DET) {
+                            if (w[c] != 0.f) {
+                                const size_t row = slab_off - (size_t)sub * VEC + off[c] + (size_t)sub;
+#pragma unroll
+                                for (int k = 0; k < VEC; ++k)
+                                    det_add(ds, det_acc + kDetHeaderWords, grad_value, row + (size_t)k * LPR,
+                                            det_contrib(w[c], gt[k]));
+                            }
+                        } else if constexpr (MIXED) {        // predicated, branch-free: bf16 result row or fp32 scratch row
                             const bool nz = w[c] != 0.f;
                             red_add_mixed(nz && fine, grad_value_bf16 + slab_off + off[c], nz && !fine, gbase + off[c],
                                           w[c] * g[0], w[c] * g[1], w[c] * g[2], w[c] * g[3]);

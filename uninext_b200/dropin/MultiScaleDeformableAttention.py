@@ -7,13 +7,15 @@ The reference builds a pybind11 extension with this name (ops/setup.py:53, ops/s
 
 Exports exactly the reference's two functions with the reference's signatures, checks and error type
 (``RuntimeError``; ops/src/ms_deform_attn.h:19-62, ops/src/cuda/ms_deform_attn_cuda.cu:28-52,93-116).
-Beyond the reference: bfloat16 ``value`` is accepted (sampling locations / attention weights are then taken as fp32).
+Beyond the reference: bfloat16 ``value`` is accepted (sampling locations / attention weights are then taken as fp32),
+and the backward honours ``torch.use_deterministic_algorithms(True)`` (``uninext_b200.determinism``): fp32 / bf16 take the
+bit-reproducible kernels, fp64 raises (or warns under ``warn_only``) and runs the normal kernels.
 """
 from __future__ import annotations
 
 import torch
 
-from uninext_b200 import _cabi
+from uninext_b200 import _cabi, determinism
 
 __all__ = ["ms_deform_attn_forward", "ms_deform_attn_backward"]
 
@@ -120,6 +122,10 @@ def ms_deform_attn_backward(value, spatial_shapes, level_start_index, sampling_l
         gv_dtype = torch.float32 if (value.dtype == torch.bfloat16 and grad_value_dtype == torch.float32) else value.dtype
         return [torch.zeros(value.shape, dtype=gv_dtype, device=value.device), torch.zeros_like(sampling_loc),
                 torch.zeros_like(attn_weight)]
+    det = determinism.mode() != determinism.OFF
+    if det and value.dtype == torch.float64:
+        determinism.alert_not_deterministic("ms_deform_attn_backward with float64 value")
+        det = False
     lib = _cabi.load()
     with torch.cuda.device(value.device):
         grad_loc = torch.empty_like(sampling_loc)
@@ -127,7 +133,20 @@ def ms_deform_attn_backward(value, spatial_shapes, level_start_index, sampling_l
         stream = torch.cuda.current_stream().cuda_stream
         common = (grad_output.data_ptr(), value.data_ptr(), spatial_shapes.data_ptr(), level_start_index.data_ptr(),
                   sampling_loc.data_ptr(), attn_weight.data_ptr(), *dims)
-        if value.dtype == torch.bfloat16:
+        if det:            # bit-reproducible grad_value: 64-bit fixed-point sums in `acc` (zero-filled by the callee)
+            acc = torch.empty(_cabi.DET_HEADER_WORDS + value.numel(), dtype=torch.int64, device=value.device)
+            if value.dtype == torch.bfloat16:
+                buf = torch.empty(value.shape, dtype=torch.float32, device=value.device)
+                keep_f32 = grad_value_dtype == torch.float32
+                grad_value = buf if keep_f32 else torch.empty_like(value)
+                code = lib.msda_backward_det_bf16(*common, acc.data_ptr(), buf.data_ptr(),
+                                                  None if keep_f32 else grad_value.data_ptr(), grad_loc.data_ptr(),
+                                                  grad_attn.data_ptr(), stream)
+            else:
+                grad_value = torch.empty_like(value)
+                code = lib.msda_backward_det_f32(*common, acc.data_ptr(), grad_value.data_ptr(), grad_loc.data_ptr(),
+                                                 grad_attn.data_ptr(), stream)
+        elif value.dtype == torch.bfloat16:
             acc = torch.empty(value.shape, dtype=torch.float32, device=value.device)
             keep_f32 = grad_value_dtype == torch.float32
             grad_value = acc if keep_f32 else torch.empty_like(value)

@@ -19,7 +19,7 @@ import torch
 from torch.autograd import Function
 from torch.autograd.function import once_differentiable
 
-from uninext_b200 import _cabi
+from uninext_b200 import _cabi, determinism
 
 
 def _stream():
@@ -30,14 +30,24 @@ def _f32c(t):
     return t.contiguous() if t.dtype == torch.float32 else t.float().contiguous()
 
 
+def _det_scratch(nbytes, device):
+    return torch.empty(nbytes // 4, dtype=torch.float32, device=device)
+
+
 def colsum(x2d: torch.Tensor) -> torch.Tensor:
     """sum over rows of a contiguous fp32 [rows, cols] CUDA tensor (cols % 4 == 0)."""
     rows, cols = x2d.shape
     if cols % 4 or x2d.data_ptr() % 16:
         return x2d.sum(0)
     out = torch.empty(cols, dtype=torch.float32, device=x2d.device)
+    lib = _cabi.load()
     with torch.cuda.device(x2d.device):
-        _cabi.check(_cabi.load().msda_colsum_f32(x2d.data_ptr(), rows, cols, out.data_ptr(), _stream()), "msda_colsum_f32")
+        if determinism.mode() != determinism.OFF:          # fixed-order sum of per-CTA partial rows
+            scratch = _det_scratch(_cabi.scratch_bytes(lib.msda_colsum_det_scratch_bytes, rows, cols), x2d.device)
+            _cabi.check(lib.msda_colsum_det_f32(x2d.data_ptr(), rows, cols, scratch.data_ptr(), out.data_ptr(), _stream()),
+                        "msda_colsum_det_f32")
+        else:
+            _cabi.check(lib.msda_colsum_f32(x2d.data_ptr(), rows, cols, out.data_ptr(), _stream()), "msda_colsum_f32")
     return out
 
 
@@ -154,10 +164,18 @@ class _LinearColsum(Function):
             g2 = g2.contiguous()
             out = torch.empty_like(g2)
             gb = torch.empty(g2.shape[1], dtype=torch.float32, device=g2.device)
+            lib = _cabi.load()
             with torch.cuda.device(g2.device):
-                _cabi.check(_cabi.load().msda_relu_backward_colsum_f32(g2.data_ptr(), y.data_ptr(), g2.shape[0], g2.shape[1],
-                                                                       out.data_ptr(), gb.data_ptr(), _stream()),
-                            "msda_relu_backward_colsum_f32")
+                if determinism.mode() != determinism.OFF:
+                    scratch = _det_scratch(_cabi.scratch_bytes(lib.msda_colsum_det_scratch_bytes, g2.shape[0], g2.shape[1]),
+                                           g2.device)
+                    _cabi.check(lib.msda_relu_backward_colsum_det_f32(g2.data_ptr(), y.data_ptr(), g2.shape[0], g2.shape[1],
+                                                                      out.data_ptr(), scratch.data_ptr(), gb.data_ptr(),
+                                                                      _stream()), "msda_relu_backward_colsum_det_f32")
+                else:
+                    _cabi.check(lib.msda_relu_backward_colsum_f32(g2.data_ptr(), y.data_ptr(), g2.shape[0], g2.shape[1],
+                                                                  out.data_ptr(), gb.data_ptr(), _stream()),
+                                "msda_relu_backward_colsum_f32")
             g2 = out
         elif ctx.relu:
             g2 = torch.ops.aten.threshold_backward(g2, y, 0.0)          # masked rows have y == 0: already zeroed
@@ -307,9 +325,16 @@ class _AddLayerNorm(Function):
         dgamma = torch.empty_like(gamma)
         dbeta = torch.empty_like(gamma)
         with torch.cuda.device(z.device):
-            _cabi.check(lib.msda_layernorm_backward_f32(gy2.data_ptr(), z.data_ptr(), gamma.data_ptr(), mean.data_ptr(),
-                                                        rstd.data_ptr(), rows, cols, dz.data_ptr(), dgamma.data_ptr(),
-                                                        dbeta.data_ptr(), _stream()), "msda_layernorm_backward_f32")
+            if determinism.mode() != determinism.OFF:
+                scratch = _det_scratch(_cabi.scratch_bytes(lib.msda_layernorm_backward_det_scratch_bytes, rows, cols), z.device)
+                _cabi.check(lib.msda_layernorm_backward_det_f32(gy2.data_ptr(), z.data_ptr(), gamma.data_ptr(), mean.data_ptr(),
+                                                                rstd.data_ptr(), rows, cols, dz.data_ptr(), scratch.data_ptr(),
+                                                                dgamma.data_ptr(), dbeta.data_ptr(), _stream()),
+                            "msda_layernorm_backward_det_f32")
+            else:
+                _cabi.check(lib.msda_layernorm_backward_f32(gy2.data_ptr(), z.data_ptr(), gamma.data_ptr(), mean.data_ptr(),
+                                                            rstd.data_ptr(), rows, cols, dz.data_ptr(), dgamma.data_ptr(),
+                                                            dbeta.data_ptr(), _stream()), "msda_layernorm_backward_f32")
         dz = dz.view(gy.shape)
         da = dz.to(ctx.a_dtype) if ctx.a_dtype != dz.dtype else dz
         db = (dz.to(ctx.b_dtype) if ctx.b_dtype != dz.dtype else dz) if ctx.has_b else None

@@ -21,7 +21,7 @@ from torch import nn
 from torch.autograd import Function
 from torch.autograd.function import once_differentiable
 
-from uninext_b200 import _cabi
+from uninext_b200 import _cabi, determinism
 
 from .deformable_transformer import MLP
 
@@ -113,9 +113,18 @@ class _DynamicMaskHead(Function):
         g = g.contiguous().float()
         gf, gp, gr = torch.empty_like(feats), torch.empty_like(params), torch.empty_like(refs)
         with torch.cuda.device(feats.device):
-            _cabi.check(lib.msda_condinst_backward_f32(g.data_ptr(), feats.data_ptr(), params.data_ptr(), refs.data_ptr(),
-                                                       inst_start.data_ptr(), n, h, w, i, max_inst, stride, rel, gf.data_ptr(),
-                                                       gp.data_ptr(), gr.data_ptr(), _stream()), "msda_condinst_backward_f32")
+            if determinism.mode() != determinism.OFF:      # per-chunk / per-warp partials summed in a fixed order
+                nbytes = _cabi.scratch_bytes(lib.msda_condinst_backward_det_scratch_bytes, n, h, w, i, max_inst)
+                scratch = torch.empty(max(nbytes // 4, 1), dtype=torch.float32, device=feats.device)
+                _cabi.check(lib.msda_condinst_backward_det_f32(g.data_ptr(), feats.data_ptr(), params.data_ptr(),
+                                                               refs.data_ptr(), inst_start.data_ptr(), n, h, w, i, max_inst,
+                                                               stride, rel, scratch.data_ptr(), gf.data_ptr(), gp.data_ptr(),
+                                                               gr.data_ptr(), _stream()), "msda_condinst_backward_det_f32")
+            else:
+                _cabi.check(lib.msda_condinst_backward_f32(g.data_ptr(), feats.data_ptr(), params.data_ptr(), refs.data_ptr(),
+                                                           inst_start.data_ptr(), n, h, w, i, max_inst, stride, rel,
+                                                           gf.data_ptr(), gp.data_ptr(), gr.data_ptr(), _stream()),
+                            "msda_condinst_backward_f32")
         return gf, gp, gr, None, None, None, None
 
 
